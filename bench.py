@@ -9,7 +9,11 @@ fingerprints resident in HBM; `e2e` = the same through the public API with HOST 
 and D2H of the ids inside the timed region).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload butina|etkdg_mmff]
+                    [--dump-outputs DIR]
     torchrun --nproc-per-node N bench.py --gpus N ...     (one rank per GPU; rank 0 prints the JSON line)
+
+--dump-outputs DIR writes what the last timed step of each leg returned as DIR/<name>.npy (see write_dumps); the inputs
+are seeded, so two builds run with the same arguments can be compared output for output.
 """
 
 from __future__ import annotations
@@ -88,6 +92,23 @@ class ClockSampler:
                     reasons.add(name)
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": sorted(reasons), "samples": len(self.rows)}
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_SAMPLE = 1 << 20  # entries of the materialised cross-similarity sampled into the dump
+DUMP_CONFORMERS = 4096  # conformer slots whose coordinates are sampled into the dump
+
+
+def write_dumps(out_dir: str, arrays: dict) -> None:
+    """--dump-outputs: one DIR/<name>.npy per array, integer and float32 outputs as float32 (exact below 2^24), float64
+    outputs as float64. Large outputs enter as fixed, seeded samples so that the whole dump stays under 64 MB."""
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float64 if v.dtype == np.float64 else np.float32) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total / 2**20:.1f} MB of outputs at this size, more than {DUMP_LIMIT_BYTES >> 20} MB")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def measured_peaks() -> tuple[float, str]:
@@ -192,14 +213,17 @@ def run_b200(args) -> None:
         _lib.set_option("similarity_pipeline_chunks", args.pipeline_chunks)
     if args.superpose_auto >= 0:
         _lib.set_option("similarity_superpose_auto", args.superpose_auto)
+    dumps = {}
     if args.workload == "conformers":
-        legs = run_conformer_legs(args, pool, dev, world, rank)
+        legs = run_conformer_legs(args, pool, dev, world, rank, dumps)
         if rank == 0:
             line = dict(legs["etkdg_mmff"])
-            line.update({"steps": 1, "warmup": 1, "higher_is_better": True, "vs_baseline": None, "data": "synthetic",
+            line.update({"warmup": 1, "higher_is_better": True, "vs_baseline": None, "data": "synthetic",
                          "config4_mmff": legs.get("config4_mmff"), "config5_etkdg_mmff": legs.get("config5_etkdg_mmff"),
                          "pool_generation_s": t_pool})
             _attach_conformer_cpu_baseline(line, pool, args)
+            if args.dump_outputs:
+                write_dumps(args.dump_outputs, dumps)
             print(json.dumps(line))
         if world > 1:
             dist.destroy_process_group()
@@ -302,6 +326,10 @@ def run_b200(args) -> None:
                      "roofline": {"bound": "hbm", "achieved": bytes_c / (ms_c * 1e-3) / 1e9, "peak": peak_c, "unit": "GB/s",
                                   "frac": bytes_c / (ms_c * 1e-3) / 1e9 / peak_c, "algorithmic_bytes": bytes_c,
                                   "kernel": "simTensorKernel<materialise> (cross_tc)", "peak_source": src_c}}
+        rng = np.random.default_rng(synthetic.SEED)
+        ri = torch.from_numpy(rng.integers(0, res.torch().shape[0], DUMP_SAMPLE)).to(dev)
+        ci = torch.from_numpy(rng.integers(0, res.torch().shape[1], DUMP_SAMPLE)).to(dev)
+        dumps["cross_tanimoto_sample"] = res.torch()[ri, ci].cpu().numpy()
         del res
         # BASELINE config 1: 1k x 1k (whole call through the public function, CUDA events on the current stream)
         ya, yb = d_fp[:1000], d_fp[1000:2000]
@@ -310,18 +338,20 @@ def run_b200(args) -> None:
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(50):
-            crossTanimotoSimilarity(ya, yb)
+            res1 = crossTanimotoSimilarity(ya, yb)
         e1.record()
         torch.cuda.synchronize()
         ms1 = e0.elapsed_time(e1) / 50
+        dumps["cross_tanimoto_1k_x_1k"] = res1.numpy()
         if cross is not None:
             cross["config1_1k_x_1k"] = {"ms_per_call": ms1, "pairs_per_s": 1e6 / (ms1 * 1e-3),
                                         "algorithmic_GBps": (8.0e6 + 256.0 * 2000) / (ms1 * 1e-3) / 1e9}
 
     # second half of the BASELINE metric: ETKDG + MMFF mols/s on config 3 (and configs 4 / 5 on eight GPUs)
-    legs = run_conformer_legs(args, pool, dev, world, rank) if pool is not None else {}
+    legs = run_conformer_legs(args, pool, dev, world, rank, dumps) if pool is not None else {}
 
     ids_h = ids.cpu().numpy()
+    dumps["butina_cluster_ids"], dumps["butina_centroids"] = ids_h, cen.cpu().numpy()
     n_clusters = int(cen.numel())
     assert ids_h.min() == 0 and ids_h.max() == n_clusters - 1
     sizes = np.bincount(ids_h, minlength=n_clusters)
@@ -424,6 +454,8 @@ def run_b200(args) -> None:
     if out["etkdg_mmff"] is not None:
         out["etkdg_mmff"]["pool_generation_s"] = t_pool
         _attach_conformer_cpu_baseline(out["etkdg_mmff"], pool, args)
+    if args.dump_outputs:
+        write_dumps(args.dump_outputs, dumps)
     print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()
@@ -564,8 +596,9 @@ def measured_traffic() -> dict:
         return {}
 
 
-def run_conformer_legs(args, pool, dev, world, rank):
-    """Configs 3 (always), 4 and 5 (8 GPUs, or --all-configs) of BASELINE.json. Returns the dict for the JSON line."""
+def run_conformer_legs(args, pool, dev, world, rank, dumps):
+    """Configs 3 (always), 4 and 5 (8 GPUs, or --all-configs) of BASELINE.json. Returns the dict for the JSON line and
+    puts this rank's config-3 results into `dumps`."""
     import torch
 
     from nvmolkit_b200 import _lib
@@ -583,15 +616,35 @@ def run_conformer_legs(args, pool, dev, world, rank):
     ids3 = (np.arange(n3) % n_pool).astype(np.int32)
     warm = ids3[:: max(1, n3 // max(1, 512 * world))]  # a short warm-up on a strided subset (allocator, clocks, caches)
     leg.step(warm, args.confs)
-    _lib.stats_read(reset=True)
-    l0 = _lib.launch_count()
-    ms, (raw, res) = _event_timed(lambda: leg.step(ids3, args.confs), dev, world)
+    # --steps counts the steps of the line's headline; beside the Butina headline this leg (tens of seconds a step) runs
+    # one. Every step is timed on its own; launches, work counters and phases are those of the last step.
+    steps = args.steps if args.workload == "conformers" else 1
+    step_ms = []
+    for _ in range(steps):
+        _lib.stats_read(reset=True)
+        l0 = _lib.launch_count()
+        ms, (raw, res) = _event_timed(lambda: leg.step(ids3, args.confs), dev, world)
+        step_ms.append(ms)
+    ms = float(np.mean(step_ms))
     launches = _lib.launch_count() - l0
     stats = _lib.stats_read(reset=True)
     phases = {"etkdg": _lib.profile_read("etkdg"), "bfgs": _lib.profile_read("bfgs")}
     ok = raw.ok.cpu().numpy().astype(bool)
     st = res.status.cpu().numpy()
     it = res.iters.cpu().numpy()
+    # a slot that failed to embed holds no conformer (its energy and coordinates are undefined): the dump keeps the
+    # per-slot embedded flag, and energies and sampled coordinates of the embedded slots only
+    embedded = np.nonzero(ok)[0]
+    dumps["etkdg_mmff_slot_mol"] = raw.slot_mol
+    dumps["etkdg_mmff_embedded"] = ok
+    dumps["etkdg_mmff_energies"] = res.energies.cpu().numpy()[embedded]
+    from nvmolkit_b200._hostutil import rows_of
+    from nvmolkit_b200.synthetic import SEED
+
+    pick = np.sort(np.random.default_rng(SEED).choice(embedded, min(len(embedded), DUMP_CONFORMERS), replace=False))
+    rows = rows_of(raw.slot_atom_start, pick)
+    dumps["etkdg_mmff_coords_sample"] = res.positions.reshape(-1, 3)[torch.from_numpy(rows).to(dev)].cpu().numpy()
+    dumps["etkdg_mmff_coords_sample_slots"] = pick
 
     # end to end through the public API: host term tables in (uploaded inside the timed region), coordinates and energies
     # out to pinned host memory
@@ -608,13 +661,13 @@ def run_conformer_legs(args, pool, dev, world, rank):
         torch.cuda.current_stream().synchronize()
         return rs
 
-    ms_e2e, _ = _event_timed(e2e_step, dev, world)
+    ms_e2e = float(np.mean([_event_timed(e2e_step, dev, world)[0] for _ in range(steps)]))
     h2d = flat.nbytes() + mmff.nbytes()
     # (the ncu traffic capture is of THIS workload at its default size on one GPU: not quoted for anything else)
     roof = _conformer_roofline(stats, phases, peak, peak_src, traffic if (n3 == 10000 and args.confs == 10 and world == 1) else {})
     out["etkdg_mmff"] = {
-        "metric": "etkdg_mmff_mols_per_s", "value": n3 / (ms * 1e-3), "unit": "mols/s", "ms_per_step": ms, "n_gpus": world,
-        "scaling": "strong",
+        "metric": "etkdg_mmff_mols_per_s", "value": n3 / (ms * 1e-3), "unit": "mols/s", "ms_per_step": ms, "steps": steps,
+        "n_gpus": world, "scaling": "strong",
         "dtype": "f64 energies / gradients / line search; inverse Hessian f32 in the embedder (option etkdg_hessian_fp64: f64, "
                  "measured beside it under embedder_hessian_f32_vs_f64), f64 in MMFF",
         "config": {"workload": f"config 3: {n3} drug-like pseudo-mols ({min(n3, n_pool)} distinct, 20-50 heavy atoms + H, mean "
@@ -742,7 +795,12 @@ def main() -> None:
     ap.add_argument("--all-configs", action="store_true", help="run configs 4 and 5 on fewer than 8 GPUs too")
     ap.add_argument("--mmff-mols", type=int, default=100000, help="config 4 size")
     ap.add_argument("--e2e-mols", type=int, default=1000000, help="config 5 size")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step of each leg returned as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
